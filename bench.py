@@ -215,7 +215,13 @@ def main():
     ap.add_argument("--chain-blocks", type=int, default=1_000_000)
     ap.add_argument("--cpu-sample", type=int, default=60000)
     ap.add_argument("--no-extra", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (one process, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl ours in a single process")
     if args.impl == "reference":
         return run_reference(args)
     if args.warmup < 3:
@@ -309,6 +315,8 @@ def main():
     barrier()
     wall = time.perf_counter() - wall0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:                              # before anything else scans: the device still holds the last step's lists
+        dump_outputs(args.dump_outputs, corpus, nq, totals, lib, _abi)
     step_ms = allmax(wall * 1e3 / args.steps)         # wall between barriers, max over ranks (includes the exchange)
     dev_step_ms = allmax(dev_ms / args.steps)         # CUDA-event time of the scan calls
     total_entries = allsum(float(args.entries))
@@ -423,6 +431,36 @@ def batch_cfg2_program(n_total: int):
         Cond(C_BODY, pattern=Pattern("regex", r"react|angular", re.IGNORECASE)),
     ])
     return pb.build()
+
+
+DUMP_SAMPLE = 1 << 17
+
+
+def dump_outputs(out_dir, corpus, nq, totals, lib, _abi):
+    """What the last timed step hands its caller, as float64 .npy files (every value is an integer below 2**53):
+      hit_counts                 [nq]     hits per query
+      hit_list_checksums         [nq, 4]  order-sensitive checksums (A, S) of each ordered hit list, in 32-bit halves: A hi, A lo, S hi, S lo
+      hit_list_sample_positions  [K]      a fixed seeded sample of K list positions
+      hit_list_sample            [nq, K]  the record index at each sampled position of each ordered list, -1 past its end
+    The full lists (about 2.5 GB at 10 M entries) are reduced to checksums plus the sample: about 34 MB in all."""
+    os.makedirs(out_dir, exist_ok=True)
+    counts = np.asarray(totals[:nq], dtype=np.uint64)
+    a, s = corpus.list_checksums(nq)
+    lo = np.uint64(0xFFFFFFFF)
+    checks = np.stack([a >> np.uint64(32), a & lo, s >> np.uint64(32), s & lo], axis=1)
+    lists = [np.empty(max(1, int(c)), dtype=np.uint64) for c in counts]
+    ptrs = (C.c_void_p * 32)(*[lst.ctypes.data for lst in lists])
+    cap = np.zeros(32, dtype=np.uint64)
+    cap[:nq] = counts
+    _abi.check(lib.fei_scan_fetch_hits(corpus.handle, nq, ptrs, _abi.ptr(cap)))   # copies the resident lists; no scan
+    pos = np.sort(np.random.default_rng(SEED).choice(corpus.n, size=min(DUMP_SAMPLE, corpus.n), replace=False))
+    sample = np.full((nq, pos.size), -1.0)
+    for q in range(nq):
+        inside = pos < int(counts[q])
+        sample[q, inside] = lists[q][pos[inside]]
+    del lists
+    for name, arr in (("hit_counts", counts), ("hit_list_checksums", checks), ("hit_list_sample_positions", pos), ("hit_list_sample", sample)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(arr, dtype=np.float64))
 
 
 def run_parity(args, rank, world, dist, corpus, prog, nq, lib, _abi):

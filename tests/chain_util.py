@@ -41,3 +41,16 @@ def expected(case):
     idx = int(words[2])
     kind = 1 if "invalid hash" in case["log"] else 2
     return False, idx, kind
+
+
+def chainsearch_golden():
+    """tests/golden/chainsearch_golden.json with every block body in place: a body stored as `"content_synth": i` is the body of
+    seeded record i (see tests/golden/make_golden_chainsearch.py)."""
+    from tests.conftest import load_golden
+    g = load_golden("chainsearch_golden.json")
+    for b in g["blocks"]:
+        md = b["memory_data"]
+        if "content_synth" in md:
+            body = synth.record(g["synth_seed"], md.pop("content_synth"))["body"].decode()
+            b["memory_data"] = {"content": body, **md}
+    return g

@@ -1,10 +1,11 @@
 #!/usr/bin/env python3
-"""Regenerate the golden fixtures by running the UNMODIFIED reference (/root/reference).
+"""Regenerate the golden fixtures by running the UNMODIFIED reference: a checkout of
+github.com/david-strejc/fei, whose path FEI_REFERENCE gives.
 
-Only runs in the build container (the reference tree does not travel to the GPU box);
-the JSON fixtures it writes are committed.  Usage:
+Needs that checkout and a built libfeiscan (the seeded record generator); the JSON fixtures
+it writes are committed, so the tests never need the reference.  Usage:
 
-    TZ=UTC python tests/golden/make_golden.py [chain] [memdir] [chainsearch]
+    FEI_REFERENCE=/path/to/fei TZ=UTC python tests/golden/make_golden.py [chain] [memdir] [chainsearch] [dropin]
 
 The reference is imported with cwd = a scratch directory (memdir_tools.utils binds
 MEMDIR_BASE to os.getcwd() at import, utils.py:16) and HOME = scratch (memorychain.py:49-52).
@@ -23,13 +24,15 @@ import threading
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+REF = os.environ.get("FEI_REFERENCE", "")
 
 sys.dont_write_bytecode = True
 os.environ.setdefault("TZ", "UTC")
 
 
 def import_reference(scratch: str):
+    if not REF or not os.path.isdir(os.path.join(REF, "memdir_tools")):
+        sys.exit("set FEI_REFERENCE to a checkout of the reference (a directory with memdir_tools/)")
     os.environ["HOME"] = scratch
     os.chdir(scratch)
     if REF not in sys.path:
@@ -178,8 +181,42 @@ def make_chain(scratch: str):
     print("wrote chain_kats.json:", len(out["single"]), "single blocks,", len(out["chains"]), "chains")
 
 
+# --------------------------------------------------------------------------- dropin
+DROPIN_MODULES = ("memdir_tools", "memdir_tools.utils", "memdir_tools.search", "memdir_tools.filter", "memdir_tools.memorychain")
+
+
+def make_dropin(scratch: str):
+    """The shape of the package fei_b200.dropin.install() patches: per module the functions, the classes with their methods,
+    the other values it defines, and the names it imports from its sibling modules (what install() has to rebind)."""
+    import importlib
+    import inspect
+    import_reference(scratch)
+    out = {"generator": "tests/golden/make_golden.py dropin", "modules": {}}
+    for name in DROPIN_MODULES:
+        mod = importlib.import_module(name)
+        entry = {"functions": [], "classes": {}, "values": [], "imports": {}}
+        for k, v in vars(mod).items():
+            if k.startswith("__") or inspect.ismodule(v):
+                continue
+            if inspect.isfunction(v) or inspect.isclass(v):
+                if v.__module__ == name:
+                    if inspect.isclass(v):
+                        entry["classes"][k] = [m for m, f in vars(v).items() if inspect.isfunction(f)]
+                    else:
+                        entry["functions"].append(k)
+                elif v.__module__.startswith("memdir_tools."):
+                    entry["imports"][k] = v.__module__
+            elif not callable(v):
+                entry["values"].append(k)
+        out["modules"][name] = entry
+    with open(os.path.join(HERE, "dropin_layout.json"), "w") as f:
+        json.dump(out, f, indent=1)
+    print("wrote dropin_layout.json:", ", ".join(f"{m}: {len(e['functions'])} functions, {len(e['classes'])} classes"
+                                                 for m, e in out["modules"].items()))
+
+
 def main():
-    what = sys.argv[1:] or ["chain", "memdir", "chainsearch"]
+    what = sys.argv[1:] or ["chain", "memdir", "chainsearch", "dropin"]
     scratch = tempfile.mkdtemp(prefix="fei_golden_")
     try:
         if "chain" in what:
@@ -190,6 +227,8 @@ def main():
         if "chainsearch" in what:
             from make_golden_chainsearch import make_chainsearch
             make_chainsearch()
+        if "dropin" in what:
+            make_dropin(scratch)
     finally:
         os.chdir(REPO)
         shutil.rmtree(scratch, ignore_errors=True)

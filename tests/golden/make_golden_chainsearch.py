@@ -1,6 +1,9 @@
 """Chain-memory search part of make_golden.py: the reference's MemorychainConnector.search_memories / search_by_tag
 (fei/tools/memorychain_connector.py:273-362) over a fixed chain.  Only the network fetch (get_chain) is replaced by a local list;
-the search code runs unmodified."""
+the search code runs unmodified.
+
+The fixture keeps the file under 1 MB by storing a body longer than STORED_BODY_MAX characters as `"content_synth": i`, the
+index of the seeded record whose body it is; tests/chain_util.chainsearch_golden() puts the body back."""
 from __future__ import annotations
 
 import importlib.util
@@ -10,8 +13,9 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+REF = os.environ.get("FEI_REFERENCE", "")
 SEED, N = 0xFE1, 300
+STORED_BODY_MAX = 4900
 
 QUERIES = [  # (query, search_content, search_subject, search_tags)
     ("python", True, True, True), ("PYTHON", True, False, False), ("learning", False, True, False), ("docker", False, False, True),
@@ -49,6 +53,8 @@ def chain_blocks():
 
 
 def make_chainsearch():
+    if not REF:
+        sys.exit("set FEI_REFERENCE to a checkout of the reference")
     spec = importlib.util.spec_from_file_location("ref_memorychain_connector", os.path.join(REF, "fei", "tools", "memorychain_connector.py"))
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
@@ -56,13 +62,20 @@ def make_chainsearch():
     conn = object.__new__(mod.MemorychainConnector)
     conn.get_chain = lambda: blocks                                   # the HTTP fetch, nothing else
     ident = {id(b["memory_data"]): i for i, b in enumerate(blocks)}
-    out = {"generator": "tests/golden/make_golden.py chainsearch", "blocks": blocks, "queries": [], "tags": []}
+    out = {"generator": "tests/golden/make_golden.py chainsearch", "blocks": blocks, "queries": [], "tags": [], "synth_seed": SEED}
     for q, c, s, t in QUERIES:
         res = conn.search_memories(q, search_content=c, search_subject=s, search_tags=t)
         out["queries"].append({"query": q, "search_content": c, "search_subject": s, "search_tags": t, "result": [ident[id(m)] for m in res]})
     for tag in TAGS:
         res = conn.search_by_tag(tag)
         out["tags"].append({"tag": tag, "result": [ident[id(m)] for m in res]})
+    stored = []
+    for b in blocks:
+        md = b["memory_data"]
+        if 1 <= b["index"] <= N and len(md["content"]) > STORED_BODY_MAX:
+            md = {"content_synth": b["index"] - 1, **{k: v for k, v in md.items() if k != "content"}}
+        stored.append({"index": b["index"], "memory_data": md})
+    out["blocks"] = stored
     with open(os.path.join(HERE, "chainsearch_golden.json"), "w") as f:
         json.dump(out, f, indent=0, sort_keys=True)
     print("wrote chainsearch_golden.json:", len(blocks), "blocks,", len(out["queries"]), "queries,", len(out["tags"]), "tag lookups")

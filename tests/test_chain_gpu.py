@@ -276,9 +276,9 @@ def test_gpu_canonical_json_matches_reference_kats(gpu, chain_golden):
 
 def test_chain_memory_search_matches_reference(gpu):
     """ChainMemorySearch (GPU) vs the reference's MemorychainConnector.search_memories / search_by_tag goldens and the oracle."""
-    from tests.conftest import load_golden
+    from tests.chain_util import chainsearch_golden
     from fei_b200.memdir_tools.chain_search import ChainMemorySearch
-    g = load_golden("chainsearch_golden.json")
+    g = chainsearch_golden()
     idx = {id(b["memory_data"]): i for i, b in enumerate(g["blocks"])}
     cs = ChainMemorySearch(g["blocks"])
     for q in g["queries"]:

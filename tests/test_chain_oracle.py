@@ -135,8 +135,8 @@ def test_native_marshalling_equals_python_marshalling(chain_golden):
 def test_chain_memory_search_oracle_matches_reference():
     """oracle.search_chain_memories / search_chain_by_tag pinned on what the reference's MemorychainConnector returned
     (tests/golden/chainsearch_golden.json, generated by make_golden.py chainsearch)."""
-    from tests.conftest import load_golden
-    g = load_golden("chainsearch_golden.json")
+    from tests.chain_util import chainsearch_golden
+    g = chainsearch_golden()
     for q in g["queries"]:
         assert co.search_chain_memories(g["blocks"], q["query"], q["search_content"], q["search_subject"], q["search_tags"]) == q["result"], q["query"]
     for t in g["tags"]:

@@ -104,28 +104,47 @@ def test_public_signatures_match_reference():
         assert got == want, (name, got, want)
 
 
-def test_dropin_install_patches_the_reference_package():
-    """Only where the reference tree is mounted (build container): install() rebinds the three entry points of the
-    unmodified package.  (Running them needs a GPU; the patched functions are the ones the gpu suite exercises.)"""
+def _write_stand_in(root, layout):
+    """A `memdir_tools` package shaped like the reference (tests/golden/dropin_layout.json, recorded from it): the same modules,
+    functions, classes with their methods, values, and names imported between modules; every body is a placeholder."""
+    pkg = root / "memdir_tools"
+    pkg.mkdir()
+    for name, m in layout["modules"].items():
+        by_src = {}
+        for k, src in m["imports"].items():
+            by_src.setdefault(src.rpartition(".")[2], []).append(k)
+        lines = [f"from .{src} import {', '.join(names)}" for src, names in by_src.items()]
+        lines += [f"def {f}(*args, **kwargs):\n    return None" for f in m["functions"]]
+        for c, methods in m["classes"].items():
+            lines.append(f"class {c}:\n" + "".join(f"    def {f}(self, *args, **kwargs):\n        return None\n" for f in methods) + "    pass")
+        lines += [f"{v} = None" for v in m["values"]]
+        (pkg / ("__init__.py" if name == "memdir_tools" else name.rpartition(".")[2] + ".py")).write_text("\n".join(lines) + "\n")
+
+
+def test_dropin_install_patches_the_reference_package(tmp_path):
+    """install() rebinds the entry points of a package laid out like the unmodified reference, including the names other
+    modules imported before install(), and leaves everything else alone.  (Running them needs a GPU; the patched functions
+    are the ones the gpu suite exercises.)"""
     import os
     import subprocess
     import sys
-    if not os.path.isdir("/root/reference/memdir_tools"):
-        pytest.skip("reference tree not mounted")
+    from tests.conftest import load_golden
+    _write_stand_in(tmp_path, load_golden("dropin_layout.json"))
     code = (
-        "import sys, os, tempfile; d = tempfile.mkdtemp(); os.chdir(d); os.environ['HOME'] = d;"
-        "sys.path.insert(0, '/root/reference'); sys.path.insert(0, %r); sys.dont_write_bytecode = True;"
+        "import sys, os; d = sys.argv[1]; os.chdir(d); os.environ['HOME'] = d;"
+        "sys.path.insert(0, d); sys.path.insert(0, %r); sys.dont_write_bytecode = True;"
+        "import memdir_tools as P, memdir_tools.utils as U, memdir_tools.search as S, memdir_tools.filter as F, memdir_tools.memorychain as M;"
+        "parse = S.parse_search_args;"
         "import fei_b200.dropin as D; D.install();"
-        "import memdir_tools.search as S, memdir_tools.filter as F, memdir_tools.memorychain as M;"
-        "assert S.__file__.startswith('/root/reference');"
+        "assert S.__file__.startswith(d);"
         "assert S.search_memories.__module__ == 'fei_b200.dropin' and F.run_filters.__module__ == 'fei_b200.dropin';"
         "assert F.FilterManager.process_memories.__module__ == 'fei_b200.dropin' and hasattr(F, 'apply_filters');"
+        "assert F.MemoryFilter.matches.__module__ == 'fei_b200.dropin';"
         "assert M.MemoryChain.validate_chain.__module__ == 'fei_b200.memdir_tools.memorychain';"
-        "import memdir_tools as P, memdir_tools.utils as U;"
         "assert P.search_memories is S.search_memories and U.search_memories.__module__ == 'fei_b200.dropin';"   # names imported before install() are rebound
-        "q = S.parse_search_args('#python +F'); assert len(q.conditions) == 2; print('patched')"
+        "assert S.parse_search_args is parse and P.parse_search_args is parse; print('patched')"
     ) % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=120)
+    out = subprocess.run([sys.executable, "-c", code, str(tmp_path)], capture_output=True, text=True, timeout=120)
     assert out.returncode == 0 and "patched" in out.stdout, out.stderr[-2000:]
 
 

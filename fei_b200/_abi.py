@@ -66,6 +66,17 @@ class JsonCol(C.Structure):
     _fields_ = [("tag", C.c_void_p), ("uniform_tag", C.c_int32), ("num", C.c_void_p), ("str", C.c_void_p), ("str_off", C.c_void_p)]
 
 
+SORT_NONE, SORT_SLOT, SORT_NAME, SORT_NAME_UID, SORT_NAME_HOST, SORT_FLAGS, SORT_BODY, SORT_TS, SORT_WALL, SORT_KEYS = range(10)
+
+
+class SortSpec(C.Structure):
+    _fields_ = [("source", C.c_uint32), ("fallback", C.c_uint32), ("prog", C.c_void_p), ("prog_len", C.c_uint64), ("keys", C.c_void_p)]
+
+
+class SortInfo(C.Structure):
+    _fields_ = [("rounds", C.c_uint32), ("radix_passes", C.c_uint32), ("refined_rows", C.c_uint64), ("ms", C.c_float)]
+
+
 _lib: Optional[C.CDLL] = None
 _lock = threading.Lock()
 
@@ -137,6 +148,7 @@ _SIGS = {
     "fei_comm_global_lists": (C.c_int, [C.c_uint32, _P, _P]),
     "fei_scan_list_checksum": (C.c_int, [_P, C.c_uint32, _P, _P]),
     "fei_scan_fetch_hits": (C.c_int, [_P, C.c_uint32, _P, _P]),
+    "fei_sort_rows": (C.c_int, [_P, C.c_uint32, _P, _P, _U64, _P, C.c_int, _U64, _U64, _P, _P]),
 }
 EXPORTS = tuple(_SIGS)
 
@@ -197,3 +209,22 @@ def device_info() -> dict:
     sm, hbm, maj, mnr = C.c_int(), C.c_uint64(), C.c_int(), C.c_int()
     check(lib().fei_device_info(C.byref(sm), C.byref(hbm), C.byref(maj), C.byref(mnr)))
     return {"sm_count": sm.value, "hbm_bytes": hbm.value, "cc": (maj.value, mnr.value)}
+
+
+def sort_rows(corpora, row_corpus: np.ndarray, row_rec: np.ndarray, source: int, descending: bool = False, first: int = 0,
+              count: Optional[int] = None, fallback: int = SORT_NONE, prog: Optional[bytes] = None, keys: Optional[np.ndarray] = None):
+    """fei_sort_rows: (row indices at sorted positions [first, first + count), SortInfo).  `corpora`: Corpus handles;
+    row i is record row_rec[i] of corpora[row_corpus[i]]."""
+    rc = np.ascontiguousarray(row_corpus, dtype=np.uint32)
+    rr = np.ascontiguousarray(row_rec, dtype=np.uint64)
+    m = rr.size
+    first = min(max(int(first), 0), m)
+    n_out = m - first if count is None else max(0, min(int(count), m - first))
+    out = np.zeros(max(1, n_out), dtype=np.uint64)
+    hs = (C.c_void_p * max(1, len(corpora)))(*[c.handle for c in corpora])
+    keys_a = np.ascontiguousarray(keys, dtype=np.uint64) if keys is not None else None
+    spec = SortSpec(source, fallback, C.cast(C.c_char_p(prog), C.c_void_p) if prog is not None else None, len(prog) if prog is not None else 0,
+                    ptr(keys_a))
+    info = SortInfo()
+    check(lib().fei_sort_rows(hs, len(corpora), ptr(rc), ptr(rr), m, C.byref(spec), 1 if descending else 0, first, n_out, ptr(out), C.byref(info)))
+    return out[:n_out].astype(np.int64), info

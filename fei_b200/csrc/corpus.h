@@ -86,6 +86,10 @@ cudaStream_t corpus_load_stream(fei_corpus* c);   // created on first use; falls
 int build_tiles(fei_corpus* c, const uint8_t* d_body, const uint64_t* d_body_off, cudaStream_t s);
 // builds the header directory from hdr / hdr_off already on the device (hdir.cu)
 int build_header_dir(fei_corpus* c, cudaStream_t s);
+// spans of the header value slot 0 of `prog` names (dict semantics of search.py:121-132) for records d_rows[0 .. m) (device array;
+// nullptr: records 0 .. m-1): d_len[i] bytes at offset d_src[i] of the header blob, d_src[i] = ~0 when absent.  Caller holds c->mu.
+int slot_spans_rows(fei_corpus* c, const uint8_t* prog, uint64_t prog_len, const uint64_t* d_rows, uint64_t m, uint32_t* d_len, uint64_t* d_src,
+                    cudaStream_t s);
 int exclusive_scan_u32_u64(const uint32_t* in, uint64_t n, uint64_t* out, DevBuf& tmp, cudaStream_t s);
 // Hook of a chunked scan: on_chunk is called on the host right after the work that makes the hit masks of records
 // [rec_begin, rec_end) final has been queued, with `side` already waiting for it; on_done after the last chunk.

@@ -1888,11 +1888,15 @@ extern "C" int fei_corpus_token_histogram(fei_corpus* c, const uint8_t* prog, ui
 // dateutil.parser.parse per record), the host needs the VALUE the reference would read for every record: slot 0 of the program
 // resolved with the reference's dict semantics (mode 0: first key whose lower() equals the field, last line of that exact key;
 // mode 1: exact key).  k_slot_spans finds the value's span in the header blob (directory walk, or the text for headers the
-// directory cannot address), k_slot_gather packs the values into one blob that goes back to the host.
+// directory cannot address), k_slot_gather packs the values into one blob that goes back to the host.  The sort keys of
+// fei_sort_rows (order.cu) read the same spans for a list of records (slot_spans_rows).
 namespace fei {
-__global__ void __launch_bounds__(256) k_slot_spans(HeadArgs a, uint32_t* __restrict__ len_out, uint64_t* __restrict__ src_out) {
-  const uint64_t rec = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
-  if (rec >= a.n) return;
+// rows == nullptr: records 0 .. m-1; else records rows[0 .. m).  Out: len_out[i], src_out[i] (offset into the header blob, ~0: absent).
+__global__ void __launch_bounds__(256) k_slot_spans(HeadArgs a, const uint64_t* __restrict__ rows, uint64_t m, uint32_t* __restrict__ len_out,
+                                                   uint64_t* __restrict__ src_out) {
+  const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+  if (i >= m) return;
+  const uint64_t rec = rows ? rows[i] : i;
   const fei_prog_hdr* ph = reinterpret_cast<const fei_prog_hdr*>(a.prog);
   const fei_prog_slot* slots = reinterpret_cast<const fei_prog_slot*>(a.prog + ph->off_slots);
   const uint32_t mode = slots[0].mode;
@@ -1942,8 +1946,8 @@ __global__ void __launch_bounds__(256) k_slot_spans(HeadArgs a, uint32_t* __rest
       p = eol + 1;
     }
   }
-  len_out[rec] = have ? vlen : 0u;
-  src_out[rec] = have ? hoff + voff : ~0ull;                     // ~0: the record has no such header
+  len_out[i] = have ? vlen : 0u;
+  src_out[i] = have ? hoff + voff : ~0ull;                       // ~0: the record has no such header
 }
 
 __global__ void __launch_bounds__(256) k_slot_gather(const uint8_t* __restrict__ hdr, const uint32_t* __restrict__ len, const uint64_t* __restrict__ src,
@@ -1959,6 +1963,26 @@ __global__ void __launch_bounds__(256) k_slot_gather(const uint8_t* __restrict__
 }
 }  // namespace fei
 
+namespace fei {
+int slot_spans_rows(fei_corpus* c, const uint8_t* prog, uint64_t prog_len, const uint64_t* d_rows, uint64_t m, uint32_t* d_len, uint64_t* d_src,
+                    cudaStream_t s) {
+  FEI_TRY(check_prog(prog, prog_len));
+  fei_prog_hdr h; memcpy(&h, prog, sizeof(h));
+  if (h.n_slots < 1) { set_error("program has no header field"); return FEI_E_BADARG; }
+  if (m == 0) return FEI_OK;
+  FEI_TRY(c->prog.ensure(prog_len + 16));
+  FEI_CUDA(cudaMemcpyAsync(c->prog.p, prog, prog_len, cudaMemcpyHostToDevice, s));
+  FEI_TRY(c->key_lut.ensure(kKeySlots * sizeof(uint32_t)));
+  k_key_lut<<<kKeySlots / 128, 128, 0, s>>>(c->prog.as<uint8_t>(), c->hdr.as<uint8_t>(), c->key_tag.as<unsigned long long>(),
+                                            c->key_rep.as<unsigned long long>(), c->key_len.as<uint32_t>(), c->key_lut.as<uint32_t>());
+  HeadArgs a{c->prog.as<uint8_t>(), c->hdr.as<uint8_t>(), c->hdr_off.as<uint64_t>(), nullptr, nullptr, nullptr, c->wall.as<int64_t>(), c->flags8.as<uint64_t>(),
+             c->fsb.as<uint32_t>(), c->n, nullptr, c->hdir.as<uint2>(), c->hdir_off.as<uint64_t>(), c->key_lut.as<uint32_t>(), false, nullptr, nullptr, nullptr, c->ts.as<int64_t>(), {}};
+  k_slot_spans<<<(unsigned)((m + 255) / 256), 256, 0, s>>>(a, d_rows, m, d_len, d_src);
+  FEI_CUDA(cudaGetLastError());
+  return FEI_OK;
+}
+}  // namespace fei
+
 /* prog: any program whose slot 0 names the field (conditions are ignored).  Out: present[n], off[n+1] (value i =
  * blob[off[i] .. off[i+1]), empty for absent headers).  FEI_E_CAPACITY with the needed size in off[n] when blob_cap is too small. */
 extern "C" int fei_corpus_slot_values(fei_corpus* c, const uint8_t* prog, uint64_t prog_len, uint8_t* present, uint64_t* off,
@@ -1967,24 +1991,14 @@ extern "C" int fei_corpus_slot_values(fei_corpus* c, const uint8_t* prog, uint64
   std::lock_guard<std::mutex> lock(c->mu);
   FEI_TRY(require_ready());
   if (!c->loaded) { set_error("corpus not loaded"); return FEI_E_STATE; }
-  FEI_TRY(check_prog(prog, prog_len));
-  fei_prog_hdr h; memcpy(&h, prog, sizeof(h));
-  if (h.n_slots < 1) { set_error("program has no header field"); return FEI_E_BADARG; }
   const uint64_t n = c->n;
+  cudaStream_t s = ctx().stream;
+  DevBuf d_len, d_src, d_off, d_present, d_out;
+  FEI_TRY(d_len.alloc(n * 4 + 4)); FEI_TRY(d_src.alloc(n * 8 + 8)); FEI_TRY(d_off.alloc((n + 1) * 8)); FEI_TRY(d_present.alloc(n + 1));
+  FEI_TRY(slot_spans_rows(c, prog, prog_len, nullptr, n, d_len.as<uint32_t>(), d_src.as<uint64_t>(), s));
   off[0] = 0;
   if (n == 0) return FEI_OK;
-  cudaStream_t s = ctx().stream;
-  FEI_TRY(c->prog.ensure(prog_len + 16));
-  FEI_CUDA(cudaMemcpyAsync(c->prog.p, prog, prog_len, cudaMemcpyHostToDevice, s));
-  FEI_TRY(c->key_lut.ensure(kKeySlots * sizeof(uint32_t)));
-  k_key_lut<<<kKeySlots / 128, 128, 0, s>>>(c->prog.as<uint8_t>(), c->hdr.as<uint8_t>(), c->key_tag.as<unsigned long long>(),
-                                            c->key_rep.as<unsigned long long>(), c->key_len.as<uint32_t>(), c->key_lut.as<uint32_t>());
-  HeadArgs a{c->prog.as<uint8_t>(), c->hdr.as<uint8_t>(), c->hdr_off.as<uint64_t>(), nullptr, nullptr, nullptr, c->wall.as<int64_t>(), c->flags8.as<uint64_t>(),
-             c->fsb.as<uint32_t>(), n, nullptr, c->hdir.as<uint2>(), c->hdir_off.as<uint64_t>(), c->key_lut.as<uint32_t>(), false, nullptr, nullptr, nullptr, c->ts.as<int64_t>(), {}};
-  DevBuf d_len, d_src, d_off, d_present, d_out;
-  FEI_TRY(d_len.alloc(n * 4)); FEI_TRY(d_src.alloc(n * 8)); FEI_TRY(d_off.alloc((n + 1) * 8)); FEI_TRY(d_present.alloc(n));
   const unsigned grid = (unsigned)((n + 255) / 256);
-  k_slot_spans<<<grid, 256, 0, s>>>(a, d_len.as<uint32_t>(), d_src.as<uint64_t>());
   FEI_TRY(exclusive_scan_u32_u64(d_len.as<uint32_t>(), n, d_off.as<uint64_t>(), c->scan_tmp, s));
   FEI_CUDA(cudaMemcpyAsync(off, d_off.p, (n + 1) * 8, cudaMemcpyDeviceToHost, s));
   FEI_CUDA(cudaStreamSynchronize(s));

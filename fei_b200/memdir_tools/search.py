@@ -4,8 +4,8 @@
 ``search_memories`` keeps its signature (search.py:337) but the per-record loop
 (search.py:361-367 -> _memory_matches_query) runs as CUDA kernels over the packed corpus:
 the query is compiled to a predicate program (fei_b200.program), scanned by libfeiscan, and
-only the hits are materialised as the reference's result dicts.  Sorting and pagination stay
-on the host and operate on the hit list exactly as the reference does (search.py:369-388).
+only the hits of the requested page are materialised as the reference's result dicts: the hits are ordered by
+`sort_by` on the device (PackedMemdir.sort_page -> fei_sort_rows) with the reference's semantics (search.py:369-388).
 """
 from __future__ import annotations
 
@@ -426,38 +426,6 @@ def _scan_ranges(pm, conds: List[Cond], ranges: List[Tuple[int, int]]) -> np.nda
     return np.concatenate(parts) if parts else np.zeros(0, dtype=np.int64)
 
 
-def _get_field_value(memory: Dict[str, Any], field: str) -> Any:
-    """Host copy of the reference's field resolution, used only to sort the materialised hits (search.py:97-139)."""
-    low = field.lower()
-    meta = memory["metadata"]
-    if low == "content":
-        return memory.get("content", "")
-    if low == "flags":
-        return "".join(meta["flags"])
-    if low == "date":
-        return meta["date"]
-    if low == "id":
-        return meta["unique_id"]
-    if low in ("filename", "folder"):
-        return memory[low]
-    if low in ("status", "maildir_status"):
-        return memory["status"]
-    if field == "Status" or low in ("status_value", "state"):
-        return memory["headers"].get("Status", "")
-    for k, v in memory["headers"].items():
-        if k.lower() == low:
-            if low in _DATE_HEADERS:
-                try:
-                    return dateutil.parser.parse(v)
-                except (ValueError, TypeError):
-                    return v
-            return v
-    for k, v in meta.items():
-        if k.lower() == low:
-            return v
-    return None
-
-
 def search_memories(query: SearchQuery, folders: Optional[List[str]] = None, statuses: Optional[List[str]] = None,
                     debug: bool = False) -> List[Dict[str, Any]]:
     pm = packer.packed()
@@ -478,15 +446,13 @@ def search_memories(query: SearchQuery, folders: Optional[List[str]] = None, sta
                 break
             conds.append(item)
         hits = _scan_ranges(pm, conds or [const(True)], ranges)
-        results = pm.materialize(hits, query.include_content)
-    if query.sort_by:
-        try:
-            results.sort(key=lambda x: _get_field_value(x, query.sort_by) or "", reverse=query.sort_reverse)
-        except Exception as e:
-            print(f"Warning: Unable to sort results: {e}")
-            results.sort(key=lambda x: x["metadata"]["timestamp"], reverse=True)
-    if query.offset or query.limit:
-        start = query.offset
-        end = None if query.limit is None else start + query.limit
-        results = results[start:end]
-    return results
+        page = range(len(hits))                          # the slice of search.py:385-388, as positions in the ordered hits
+        if query.offset or query.limit:
+            start = query.offset
+            end = None if query.limit is None else start + query.limit
+            page = page[start:end]
+        if query.sort_by:                                # ordered on the device; only the page is materialised
+            hits = pm.sort_page(hits, query.sort_by, query.sort_reverse, query.include_content, page.start, len(page))
+        else:
+            hits = hits[page.start:page.stop]
+        return pm.materialize(hits, query.include_content)

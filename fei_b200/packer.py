@@ -419,6 +419,8 @@ class PackedMemdir:
         self._field_values: Dict[str, Tuple[np.ndarray, np.ndarray, List[str]]] = {}
         self.parsed_dates: Dict[str, Tuple[Any, bool]] = {}
         self._aux_next = 0
+        self._key_error: Optional[BaseException] = None
+        self.last_sort_info = None                           # fei_sort_info of the last device sort (sort_page)
         self._seg_index: Optional[Tuple[List[Tuple[str, str]], np.ndarray]] = None
         self._walk_cache: Optional[List[str]] = None
         self._tree_dirty = True
@@ -1210,6 +1212,113 @@ class PackedMemdir:
             got = self._field_values[key] = (present, inv, distinct)
         return got
 
+    # ---- result order (search.py:370-388)
+    def sort_page(self, positions: np.ndarray, field: str, reverse: bool, include_content: bool, first: int, count: int) -> np.ndarray:
+        """The listing positions of the hits (in hit order) ordered as the reference orders their dicts,
+        results.sort(key=lambda x: _get_field_value(x, field) or "", reverse=reverse) with its warning and newest-first
+        fallback (search.py:97-139, :370-382), then sliced to [first, first + count).  Keys the device can order go to
+        fei_sort_rows; the sort runs on the host only where CPython's own comparisons define the outcome: keys of more than
+        one class (str / int / naive / aware datetime), which make list.sort raise and leave a partial order, or a key that
+        raises."""
+        positions = np.asarray(positions, dtype=np.int64)
+        m = len(positions)
+        if m == 0:
+            return positions
+        low = field.lower()
+        kw: Dict[str, Any] = {}
+        if low == "content":
+            if not include_content:                                   # memory.get("content", "") == "" for every hit: order unchanged
+                return positions[first:first + count]
+            kw["source"] = _abi.SORT_BODY
+        elif low == "flags":
+            kw["source"] = _abi.SORT_FLAGS
+        elif low == "date":
+            kw["source"] = _abi.SORT_WALL                             # naive datetime.fromtimestamp: the wall clock, not ts (DST)
+        elif low == "id":
+            kw["source"] = _abi.SORT_NAME_UID
+        elif low == "filename":
+            kw["source"] = _abi.SORT_NAME
+        elif low in ("folder", "status", "maildir_status"):
+            fsb = self.arrays["fsb"][positions]
+            if low == "folder":
+                ids, names = fsb & 0xFFFF, {i: f for f, i in self.folder_ids.items()}
+            else:
+                ids, names = (fsb >> 16) & 0xFF, dict(enumerate(U.STANDARD_FOLDERS))
+            uniq, back = np.unique(ids, return_inverse=True)
+            kw.update(source=_abi.SORT_KEYS, keys=np.asarray(_ranks([names[int(u)] for u in uniq]), dtype=np.uint64)[back])
+        elif low in ("status_value", "state"):                        # headers.get("Status", ""): the exact key
+            kw.update(source=_abi.SORT_SLOT, prog=_slot_prog("Status", 1))
+        elif low in ("due", "created", "modified", "deleteddate", "timestamp"):
+            keys = self._host_keys(positions, field, low)
+            if keys is None or isinstance(keys, list):                # a key raised, or classes mix: CPython decides
+                ts = self.arrays["ts"][positions].tolist()
+                order = python_order(keys if keys is not None else [], ts, reverse, self._key_error)
+                return positions[np.asarray(order, dtype=np.int64)][first:first + count]
+            kw.update(source=_abi.SORT_KEYS, keys=keys)
+        else:
+            kw.update(source=_abi.SORT_SLOT, prog=_slot_prog(field, 0),
+                      fallback={"unique_id": _abi.SORT_NAME_UID, "hostname": _abi.SORT_NAME_HOST}.get(low, _abi.SORT_NONE))
+        if count <= 0:
+            return positions[:0]
+        corpora = self._corpora()
+        dev = self.dev[positions]
+        los = np.array([lo for _, lo in corpora], dtype=np.int64)
+        rc = np.searchsorted(los, dev, side="right") - 1
+        rows, self.last_sort_info = _abi.sort_rows([c for c, _ in corpora], rc, dev - los[rc], descending=reverse, first=first, count=count, **kw)
+        return positions[rows]
+
+    def _host_keys(self, positions: np.ndarray, field: str, low: str):
+        """Keys of a date header (dateutil.parser.parse of the value, the raw value when that fails, search.py:124-131) or of
+        `timestamp` (a header string, else the int metadata), `or ""` applied.  Returns uint64 ranks when every hit's key is of
+        one class, the list of key objects when classes mix, None when computing a key raises (self._key_error)."""
+        from .memdir_tools.search import _parse_dt
+        import dateutil.parser
+        self._key_error = None
+        present, inv, distinct = self.header_values(field)
+        inv_h = inv[positions]
+        if low == "timestamp":
+            ts_h = self.arrays["ts"][positions]
+            hdr = present[positions]
+            meta_str = ~hdr & (ts_h == 0)                             # int 0 or "" -> ""
+            classes = (bool(hdr.any() or meta_str.any())) + bool((~hdr & (ts_h != 0)).any())
+            if classes > 1 and len(positions) > 1:
+                d = distinct + [""]
+                return [d[u] if h else (t or "") for u, h, t in zip(inv_h.tolist(), hdr.tolist(), ts_h.tolist())]
+            if not hdr.any() and not meta_str.any():
+                return np.unique(ts_h, return_inverse=True)[1].astype(np.uint64)
+            texts = np.array(distinct + [""], dtype=object)
+            vals = np.where(hdr, inv_h, len(distinct))
+            uniq, back = np.unique(vals, return_inverse=True)
+            return np.asarray(_ranks([texts[u] for u in uniq]), dtype=np.uint64)[back]
+        uniq, back = np.unique(inv_h, return_inverse=True)
+        objs: List[Any] = []
+        errs: Dict[int, BaseException] = {}
+        for k, u in enumerate(uniq.tolist()):
+            if u == len(distinct):
+                objs.append("")                                       # no such header: None or "" -> ""
+                continue
+            text = distinct[u]
+            parsed = self.parsed_dates.get(text)
+            if parsed is None:
+                parsed = self.parsed_dates[text] = _parse_dt(text)
+            dt, today_dependent = parsed
+            if dt is None or today_dependent:                         # parse as the reference does: default = today
+                try:
+                    dt = dateutil.parser.parse(text)
+                except (ValueError, TypeError):
+                    dt = None
+                except Exception as e:                                # escapes _get_field_value and aborts the sort
+                    errs[k] = e
+            objs.append(dt if dt is not None else (text or ""))
+        if errs:
+            first_bad = int(np.nonzero(np.isin(back, list(errs)))[0][0])
+            self._key_error = errs[int(back[first_bad])]
+            return None
+        kinds = {_key_class(o) for o in objs}
+        if len(kinds) > 1 and len(positions) > 1:
+            return [objs[b] for b in back.tolist()]
+        return np.asarray(_ranks(objs), dtype=np.uint64)[back]
+
     def begin_query(self) -> None:
         self._aux_next = 0
 
@@ -1306,6 +1415,48 @@ class PackedMemdir:
                     c.close()
             self.corpus = self.delta = None
             self.watcher.close()
+
+
+def python_order(keys: Sequence[Any], ts: Sequence[int], reverse: bool, key_error: Optional[BaseException] = None) -> List[int]:
+    """What search.py:370-382 does to a result list, on indices: list.sort by the keys (a failed sort leaves CPython's partial
+    order, the same for indices as for the dicts), then on any exception the warning and a stable newest-first sort.
+    key_error: the exception computing a key raised (the list is then left as it was)."""
+    idx = list(range(len(ts)))
+    try:
+        if key_error is not None:
+            raise key_error
+        idx.sort(key=keys.__getitem__, reverse=reverse)
+    except Exception as e:
+        print(f"Warning: Unable to sort results: {e}")
+        idx.sort(key=ts.__getitem__, reverse=True)
+    return idx
+
+
+def _key_class(o: Any) -> str:
+    if isinstance(o, datetime):
+        return "aware" if o.tzinfo is not None and o.utcoffset() is not None else "naive"
+    return type(o).__name__
+
+
+def _ranks(objs: Sequence[Any]) -> List[int]:
+    """Dense ranks under Python's comparison (objects of one class); equal objects share a rank."""
+    order = sorted(range(len(objs)), key=objs.__getitem__)
+    out = [0] * len(objs)
+    r = 0
+    for t, i in enumerate(order):
+        if t and objs[order[t - 1]] < objs[i]:
+            r += 1
+        out[i] = r
+    return out
+
+
+def _slot_prog(field: str, mode: int) -> bytes:
+    """A program whose slot 0 names one header (mode 0: first key whose lower() equals the field; 1: the exact key)."""
+    from .program import C_SLOT, Cond, ProgramBuilder
+    from .regexc import Pattern
+    pb = ProgramBuilder()
+    pb.add_query([Cond(C_SLOT, pattern=Pattern("regex", "", re.IGNORECASE), field=field, mode=mode)])
+    return pb.build()
 
 
 def _subset(L: DirListing, sel: np.ndarray) -> DirListing:

@@ -249,6 +249,41 @@ int fei_corpus_slot_values(fei_corpus* c, const uint8_t* prog, uint64_t prog_len
                            uint8_t* blob, uint64_t blob_cap);
 int fei_corpus_set_aux(fei_corpus* c, uint32_t k, const uint8_t* bytes, uint64_t n);
 
+/* ---- result order --------------------------------------------------------------
+ * Replaces the sort and the slice of memdir_tools.search.search_memories (memdir_tools/search.py:370-388):
+ *     results.sort(key=lambda x: _get_field_value(x, sort_by) or "", reverse=sort_reverse)   (keys: search.py:97-139)
+ *     results = results[offset : offset + limit]
+ * for the keys whose order the device can decide.  Row i is record row_rec[i] of corpora[row_corpus[i]] (a base corpus and the
+ * delta of an incremental sync can be mixed); rows [0, m) are in the order the hits were found.  The sort is stable, also when
+ * descending (as CPython's reverse=True: equal keys keep their order).  out[0 .. min(count, m - first)) receives the row
+ * indices at sorted positions [first, first + count).  Key sources (spec->source):
+ *   FEI_SORT_SLOT        the header value slot 0 of spec->prog names (mode 0: first key whose lower() equals the field, dict
+ *                        semantics; mode 1: exact key); an absent header reads as spec->fallback: FEI_SORT_NONE (the empty
+ *                        string), FEI_SORT_NAME_UID or FEI_SORT_NAME_HOST (the metadata of search.py:134-137)
+ *   FEI_SORT_NAME        the file name; FEI_SORT_NAME_UID / _HOST its unique_id / hostname (corpora loaded with names)
+ *   FEI_SORT_FLAGS       the flag letters joined;  FEI_SORT_BODY the stripped body
+ *   FEI_SORT_TS / _WALL  the filename timestamp / datetime.fromtimestamp(ts) (naive wall clock)
+ *   FEI_SORT_KEYS        spec->keys[i], unsigned (values the caller ranked)
+ * Strings compare by unsigned byte (= code point order for UTF-8), a proper prefix first.  info (may be NULL): rounds = sort
+ * rounds (one per 7 bytes of the longest common prefix still tied), radix_passes, refined_rows = rows re-sorted after round 0,
+ * ms = device time from the first to the last kernel (CUDA events).  FEI_E_BADARG for a bad spec or row.          */
+enum { FEI_SORT_NONE = 0, FEI_SORT_SLOT = 1, FEI_SORT_NAME = 2, FEI_SORT_NAME_UID = 3, FEI_SORT_NAME_HOST = 4, FEI_SORT_FLAGS = 5,
+       FEI_SORT_BODY = 6, FEI_SORT_TS = 7, FEI_SORT_WALL = 8, FEI_SORT_KEYS = 9 };
+typedef struct fei_sort_spec {
+  uint32_t source;
+  uint32_t fallback;            /* FEI_SORT_SLOT only */
+  const uint8_t* prog;          /* FEI_SORT_SLOT: compiled program (fei_b200/program.py), slot 0 names the header */
+  uint64_t prog_len;
+  const uint64_t* keys;         /* FEI_SORT_KEYS: m keys */
+} fei_sort_spec;
+typedef struct fei_sort_info {
+  uint32_t rounds, radix_passes;
+  uint64_t refined_rows;
+  float ms;
+} fei_sort_info;
+int fei_sort_rows(fei_corpus* const* corpora, uint32_t n_corpora, const uint32_t* row_corpus, const uint64_t* row_rec, uint64_t m,
+                  const fei_sort_spec* spec, int descending, uint64_t first, uint64_t count, uint64_t* out, fei_sort_info* info);
+
 /* ---- Memorychain validation -----------------------------------------------------
  * Replaces the loop of MemoryChain.validate_chain (memdir_tools/memorychain.py:596-618)
  * and its inline copy in receive_chain_update (:1059-1078):
